@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- mel frames/sec of the Tacotron hot path on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--mode infer]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--mode infer] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one synthetic batch of BASELINE config 2:
 B=32 utterances, char length 128, 200 decoder steps, r=5  (32 000 mel frames), free-running
@@ -14,6 +14,8 @@ ranks; plus `e2e` (host pinned inputs -> H2D -> public API -> D2H of output + al
 --impl reference: the reference's CPU path stand-in (the PyTorch-CPU oracle port; TensorFlow 1.2
 cannot be installed here) on the same config, all host threads.
 N > 1: inference shards by utterance with no exchange -> N independent replicas (weak scaling).
+--dump-outputs DIR: after the timed steps, rank 0 writes what its last timed step returned as DIR/<name>.npy (float32,
+see dump_outputs); the inputs and weights are seeded, so two builds can be compared output for output.
 """
 import argparse
 import json
@@ -570,6 +572,23 @@ def measure_c5_isolated(args):
     return _isolated(args, "c5-worker", 240)
 
 
+DUMP_OUTPUT_SAMPLE = 8 * 1024 * 1024            # elements of `output` kept by --dump-outputs (32 MB of float32)
+
+
+def dump_outputs(out_dir, y, out, align):
+    """Write what one inference step returns to its caller as float32 .npy files: seq2seq_output [B, T, 80 r] (10 MB)
+    and alignments [B, T, Tx] (3 MB) whole; of output [B, T, 1025 r] (131 MB) the flat elements at a fixed sorted random
+    index set (torch.randperm, CPU generator seeded 0), so that all files stay under 64 MB together."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    flat = out.reshape(-1)
+    idx = torch.randperm(flat.numel(), generator=torch.Generator().manual_seed(0))[:DUMP_OUTPUT_SAMPLE].sort().values
+    arrays = {"seq2seq_output": y, "alignments": align, "output_sample": flat[idx.to(flat.device)]}
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().float().cpu().numpy())
+
+
 def run_ours(args):
     import torch
     import torch.distributed as dist
@@ -620,7 +639,7 @@ def run_ours(args):
         flush.zero_()
         model._marks = []
         starts[i].record()
-        step()
+        last = step()
         ends[i].record()
         marks = model._marks
         model._marks = None
@@ -635,6 +654,9 @@ def run_ours(args):
     launches = lib.taco_launch_count() - launches0 + args.steps * int(model.last_graph_kernels)
     clocks = sampler.stop() if sampler else None
     _log("timed steps done")
+    if args.dump_outputs and rank == 0:                  # before the e2e loop below overwrites the result buffers
+        dump_outputs(args.dump_outputs, last[0], last[1], model.alignments)
+        _log(f"outputs of the last timed step written to {args.dump_outputs}")
     total_ms = sum(s.elapsed_time(e) for s, e in zip(starts, ends))
     total_ms = D.max_over_ranks(total_ms)                 # the job advances at the slowest rank
     ms_per_step = total_ms / args.steps
@@ -644,7 +666,7 @@ def run_ours(args):
     # Every step: H2D of the step's inputs from pinned memory, Tacotron.inference, D2H of output + alignments
     # into pinned memory.  The D2H of step i runs on a copy stream and overlaps the encoder/decoder of step
     # i+1 (the result buffers are only rewritten by the decoder / post-net sections, which wait for the copy).
-    e2e_steps = max(3, args.steps)                   # same step count as the device-timed region (the last D2H is not overlapped)
+    e2e_steps = args.steps                           # same step count as the device-timed region (the last D2H is not overlapped)
     copy_stream = torch.cuda.Stream()
     ev_done = torch.cuda.Event()
     ev_align_copied, ev_out_copied = torch.cuda.Event(), torch.cuda.Event()
@@ -830,7 +852,13 @@ def main():
     ap.add_argument("--no-graph", action="store_true", help="launch kernels eagerly instead of replaying CUDA graphs")
     ap.add_argument("--no-train", action="store_true", help="skip the side measurement of the training step")
     ap.add_argument("--no-c5", action="store_true", help="skip the single-utterance + Griffin-Lim latency side measurement")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed inference step returned (rank 0) as DIR/<name>.npy, float32, < 64 MB in all")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.mode != "infer"):
+        ap.error("--dump-outputs applies to the default inference arm (--impl ours --mode infer) only")
     if args.impl == "reference":
         run_reference(args)
     elif args.impl == "reference-probe":                 # internal: child process of pick_cpu_threads
